@@ -2,7 +2,7 @@
 """bench.py — BASELINE.json metric: 3-D vol-pairs/sec (160x192x224) for one diffeomorphic VxmDense TRAINING step
 (forward + NCC/Grad losses + backward + gradient allreduce + Adam) at N GPUs, one volume pair per GPU per step.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for how each field is obtained.
 """
@@ -42,7 +42,14 @@ def parse():
     ap.add_argument("--no-parity", action="store_true", help="skip the first-step loss check against the CPU oracle and the bf16x3 parity-mode leg")
     ap.add_argument("--no-gpu-eager", action="store_true", help="skip the reference-torch-on-GPU (eager ATen / cuDNN) baseline leg")
     ap.add_argument("--no-c4", action="store_true", help="skip the BASELINE config 4 sweep (256^3 warp / VecInt GB/s)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (its loss) and left behind "
+                    "(the trained parameters) to DIR/<name>.npy, float32, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 training step (--impl b200)")
+    return args
 
 
 def load_peaks():
@@ -478,10 +485,12 @@ def b200_arm(args):
     t_host0 = time.time()
     e0.record()
     for i in range(K):
-        step(*pairs_dev[i % NPAIR])
+        loss_last = step(*pairs_dev[i % NPAIR])
     e1.record()
     barrier()
     t_host1 = time.time()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss_last, model)
     ms = e0.elapsed_time(e1)
     launches = (launches_per_step * K) if graphed else (vxm._lib.launch_count() - n0)
     ms = vdist.max_over_ranks(ms, dev)
@@ -653,6 +662,20 @@ def b200_arm(args):
                 gpu_eager_baseline=gpu_eager, c4_sweep=c4)
     print(json.dumps(line), flush=True)
     _leave(world, rank)
+
+
+def dump_outputs(out_dir, loss, model):
+    """The arrays a caller of the training step has after its last timed step: the loss it returned and the model's
+    parameters after the Adam update, one float32 .npy each (about 1.3 MB for the default U-Net, whatever the shape).
+    The inputs, the initial weights and the number of steps depend only on the arguments, so two builds run with the same
+    arguments can be compared file by file.  Gradient sums accumulated with atomics make even two runs of one build differ
+    in the last bits, and Adam magnifies that where a gradient is near zero: compare the weights with a tolerance."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = dict(loss=loss.detach().float().reshape(1))
+    arrays.update(("param." + k, p.detach().float()) for k, p in model.named_parameters())
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
 
 
 def _leave(world, rank=None):

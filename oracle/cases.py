@@ -4,9 +4,18 @@ TEST INFRASTRUCTURE ONLY.  Everything is generated with numpy's PCG64 streams an
 float32 arithmetic (adds / multiplies only, no transcendental functions), so the same
 arrays are reproduced bit for bit on the GPU box.
 """
+import hashlib
+
 import numpy as np
 
 F32 = np.float32
+
+
+def digest(a):
+    """Shape and SHA-256 of the values of `a` (widened to float64, -0.0 folded into 0.0): two float arrays have the same
+    digest exactly when np.array_equal holds, so a frozen digest stands for the array in an exact comparison."""
+    a = np.ascontiguousarray(np.asarray(a, dtype=np.float64) + 0.0)
+    return [list(a.shape), hashlib.sha256(a.tobytes()).hexdigest()]
 
 
 def _lerp_axis(x, out_n, axis):

@@ -1,10 +1,9 @@
 """Import the *unmodified* reference (voxelmorph @ /root/reference) on CPU.
 
-TEST INFRASTRUCTURE ONLY, and only usable in the build container: `/root/reference`
-does not exist on the GPU box.  It is used by `oracle/make_golden.py` to freeze the
-reference's outputs into `tests/golden/` and by `tests/test_oracle_vs_reference.py`
-(skipped when the reference tree is absent) to pin the restatements in
-`oracle/spec_np.py` / `oracle/ref_torch.py`.
+TEST INFRASTRUCTURE ONLY: used by `oracle/make_golden*.py` to freeze the reference's
+outputs into `tests/golden/`, against which the tests pin the restatements in
+`oracle/spec_np.py` / `oracle/ref_torch.py` and the product package.  The tests never
+import the reference.
 
 The reference hard-imports three packages that are absent from this image and
 irrelevant to the torch hot path (`neurite`, `skimage.measure`, `pystrum`):

@@ -13,8 +13,8 @@ pinned by the reference's setup.py) is called here through the same torch entry 
 the explicit formulas are restated separately in oracle/spec_np.py and the two are
 cross-checked in tests/.
 
-Pinned against the unmodified reference by tests/golden (oracle/make_golden.py) and,
-when /root/reference is present, live in tests/test_oracle_vs_reference.py.
+Pinned against the unmodified reference by tests/golden (oracle/make_golden.py and
+oracle/make_golden_outputs.py, checked in tests/test_oracle_vs_reference.py).
 """
 import math
 

@@ -9,8 +9,8 @@ ATen headers are cited as [torch] <header>:<line>.
 Parity status: the reference ships no tests or golden vectors ("parity unpinned" by
 the reference itself).  These restatements are pinned instead against outputs of
 the unmodified reference run in the build container (oracle/make_golden.py ->
-tests/golden/*.npz) and against the reference imported live
-(tests/test_oracle_vs_reference.py, skipped when /root/reference is absent).
+tests/golden/*.npz, oracle/make_golden_outputs.py -> tests/golden/reference_outputs.json,
+checked in tests/test_oracle_vs_reference.py).
 
 All arithmetic is float32 with one rounding per operation (numpy never contracts
 to FMA), which is what makes the nearest-neighbour index sequence reproducible

@@ -91,8 +91,18 @@ def full_cfg(kw):
     return c
 
 
+@pytest.fixture
+def golden_threads():
+    """torch's CPU convolutions split their sums by thread count, so their bits depend on it: bit-exact comparisons with
+    the vectors oracle/make_golden.py froze run with the 8 threads it used, whatever the machine's core count."""
+    prev = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(prev)
+
+
 @pytest.mark.parametrize("name", sorted(VARIANTS))
-def test_vxmdense_restatement_against_reference(golden, name):
+def test_vxmdense_restatement_against_reference(golden, golden_threads, name):
     """ref_torch.vxm_forward (functional restatement) == reference VxmDense.forward, all ctor variants."""
     g = golden("vxmdense")
     cfg = full_cfg(VARIANTS[name])

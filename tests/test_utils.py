@@ -1,9 +1,14 @@
 """CPU tests of the host-side evaluation helpers (voxelmorph_b200/utils.py, next rows N2 / N3) against the oracle
-restatements (oracle/spec_np.py) and, in the build container, the live reference (py/utils.py:265-287, :473-516)."""
+restatements (oracle/spec_np.py) and the reference's outputs (py/utils.py:265-287, :473-516) frozen into
+tests/golden/reference_outputs.json by oracle/make_golden_outputs.py."""
+import json
+import os
+
 import numpy as np
 import pytest
 
-from oracle import cases, ref_import, spec_np
+from conftest import GOLDEN
+from oracle import cases, spec_np
 
 
 def fields():
@@ -35,16 +40,11 @@ def test_jacobian_determinant_matches_oracle_and_counts_folds():
         utils.jacobian_determinant(np.zeros((4, 4, 4, 2)))
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not present")
 def test_against_live_reference():
-    import sys
     from voxelmorph_b200 import utils
-    ref = ref_import.import_reference()
-    nd_mod = sys.modules["pystrum.pynd.ndutils"]
-    if not hasattr(nd_mod, "volsize2ndgrid"):
-        nd_mod.volsize2ndgrid = lambda volshape: np.meshgrid(*[np.arange(s) for s in volshape], indexing="ij")
+    ref = json.load(open(os.path.join(GOLDEN, "reference_outputs.json")))["eval_helpers"]
     rng = np.random.RandomState(2)
     a, b = rng.randint(0, 5, size=(9, 10, 11)), rng.randint(0, 5, size=(9, 10, 11))
-    assert np.allclose(utils.dice(a, b), ref.py.utils.dice(a, b), rtol=0, atol=1e-15)
-    for d in list(fields())[:2]:
-        np.testing.assert_allclose(utils.jacobian_determinant(d), ref.py.utils.jacobian_determinant(d), rtol=0, atol=1e-12)
+    assert np.allclose(utils.dice(a, b), np.array(ref["utils_dice"]), rtol=0, atol=1e-15)
+    for d, r in zip(list(fields())[:2], ref["utils_jacdet"], strict=True):
+        np.testing.assert_allclose(utils.jacobian_determinant(d), np.array(r), rtol=0, atol=1e-12)

@@ -1,7 +1,6 @@
 """Helper script of the drop-in tests: the training loop of the reference's scripts/torch/train.py:95-233 restated on
-`import voxelmorph as vxm` (argument handling cut down to what the tests pass).  The reference tree does not exist on the
-GPU box, so the `-m gpu` tests run this body; tests/test_shim.py additionally runs the reference's own train.py / register.py
-byte for byte where /root/reference is present."""
+`import voxelmorph as vxm` (argument handling cut down to what the tests pass), run by the `-m gpu` tests of
+tests/test_shim.py."""
 import argparse
 import json
 import os
